@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json metric: Inflate GB/s (uncompressed) on 1 GiB synthetic DEFLATE @1/2/4/8 GPU vs the CPU path.
 
-  python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5] [--impl reference] [--dump-outputs DIR]
 
 Default = BASELINE config 2 (SURVEY.md 8d): 16 384 gzip members x 64 KiB of synthetic wiki-like text, one dynamic-Huffman
 block per member, ~394 MiB compressed -> 1 GiB, per GPU.  One JSON line on rank 0:
@@ -25,6 +25,9 @@ block per member, ~394 MiB compressed -> 1 GiB, per GPU.  One JSON line on rank 
              roofline, cpu_baseline and a parity check: 3 Deflate level 6 on 256 MiB, 4 BZip2Decoder on 512 MiB of 900 kB
              blocks, 5 ZipDecoder on a 1024-member 4 GiB zip.  --config K makes K the line's own metric (4 and 5 shard over
              the ranks of a torchrun job).
+  --dump-outputs DIR
+             (config 2) after the timed steps, what the last step handed its caller, as float .npy files in DIR
+             (dump_outputs): two builds run with the same arguments decode the same input and can be compared file by file.
 """
 from __future__ import annotations
 
@@ -64,6 +67,26 @@ def peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_UNITS = 128  # 128 units x 64 KiB of decoded bytes as float32: 32 MiB, so that a whole dump stays under 64 MB
+DUMP_SEED = 0xB200
+
+
+def dump_outputs(out_dir: str, full: np.ndarray, status: np.ndarray, out_len: np.ndarray, in_used: np.ndarray):
+    """--dump-outputs: the arrays one step of b200z_inflate_batch_device returns, as .npy files in out_dir.
+      status, out_len, in_used        float32 [units of this rank]; every value is below 2**24, so float32 holds it exactly
+      decoded_sample                  float32 [DUMP_UNITS, UNIT]: the decoded bytes of whole 64 KiB units of the stream
+                                      (N > 1: of the gathered stream), a fixed, seeded sample -- all of it would take 4 GiB
+      decoded_sample_units            float64 [DUMP_UNITS]: which units of the stream those are (ascending)"""
+    os.makedirs(out_dir, exist_ok=True)
+    n_total = full.size // UNIT
+    units = np.sort(np.random.default_rng(DUMP_SEED).choice(n_total, size=min(DUMP_UNITS, n_total), replace=False))
+    arrays = {"status": status.astype(np.float32), "out_len": out_len.astype(np.float32), "in_used": in_used.astype(np.float32),
+              "decoded_sample": full.reshape(n_total, UNIT)[units].astype(np.float32),
+              "decoded_sample_units": units.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -256,7 +279,7 @@ def _timed_calls(fn, reps):
     return ts
 
 
-def side_config3(L, cores):
+def side_config3(L, cores, reps=3):
     """Deflate level 6 on 256 MiB of the synthetic text through b200z_deflate_raw (host in, host out, pinned): the only
     entry point the encoder has, so value == e2e.  Parity: the first 32 MiB compressed alone are byte-identical to the
     oracle's Deflate(level: 6) of the same bytes; the full output inflates back to the input (CRC-32)."""
@@ -274,7 +297,7 @@ def side_config3(L, cores):
         assert rc == 0, _ffi.last_error()
 
     call()
-    ts = _timed_calls(call, 3)
+    ts = _timed_calls(call, reps)
     z = C.string_at(h_out, out_len.value)
     c_bytes = out_len.value
     ok_round = zlib.crc32(zlib.decompress(z, -15)) == zlib.crc32(text.tobytes()) == crc.value
@@ -314,7 +337,7 @@ def make_bz2_stream(L, text: np.ndarray):
     return zbuf[:zl.value].copy()
 
 
-def side_config4(L, cores, world=1, rank=0, dist=None):
+def side_config4(L, cores, world=1, rank=0, dist=None, reps=3):
     """BZip2Decoder(verify) on 512 MiB of text in 900 kB blocks (one BZh9 stream, written by the device encoder whose bytes
     the tests pin to the oracle's).  N = 1: b200z_bzip2_decode host -> host.  N > 1: blocks sharded over the ranks
     (shard.bzip2_decode_sharded: per-block reports exchanged, decoded bytes stay on the rank that produced them)."""
@@ -334,7 +357,7 @@ def side_config4(L, cores, world=1, rank=0, dist=None):
             assert rc == 0, _ffi.last_error()
 
         call()
-        ts = _timed_calls(call, 3)
+        ts = _timed_calls(call, reps)
         ok = ol.value == m and zlib.crc32(C.string_at(h_o, m)) == src_crc
         L.b200z_host_free(h_o)
         dt = min(ts)
@@ -345,7 +368,7 @@ def side_config4(L, cores, world=1, rank=0, dist=None):
         h_o = L.b200z_host_alloc(ocap)
         zv = (C.c_uint8 * z.size).from_address(h_z)
         ts, r = [], None
-        for i in range(4):
+        for i in range(reps + 1):
             dist.barrier()
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -400,7 +423,7 @@ def make_zip(n_members: int, size: int, stream: int = 7000):
     return data, [crc for _, crc in parts]
 
 
-def side_config5(L, cores, world=1, rank=0, dist=None):
+def side_config5(L, cores, world=1, rank=0, dist=None, reps=3):
     """ZipDecoder end to end on a 1024-member x 4 MiB synthetic .zip (method 8, a full-flush point every 64 KiB -- still one
     valid DEFLATE stream per member): b200z_zip_list + ONE b200z_zip_extract call, host in, host out.  N > 1: the members are
     packed onto the ranks (shard.pack_members), every rank extracts its share."""
@@ -430,7 +453,7 @@ def side_config5(L, cores, world=1, rank=0, dist=None):
     if world > 1:
         import torch
         ts = []
-        for i in range(3):
+        for i in range(reps + 1):
             dist.barrier()
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -441,7 +464,7 @@ def side_config5(L, cores, world=1, rank=0, dist=None):
         ts = ts[1:]
     else:
         call()
-        ts = _timed_calls(call, 3)
+        ts = _timed_calls(call, reps)
     out = np.ctypeslib.as_array((C.c_uint8 * tot).from_address(h_out))
     ok = all(s == 0 for s in st) and all(o == size for o in ol)
     ok = ok and all(zlib.crc32(out[j * size:(j + 1) * size].tobytes()) == crcs[mine[j]] for j in range(0, k, 7))
@@ -521,7 +544,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config != 2):
+        ap.error("--dump-outputs dumps the config 2 decode of the GPU arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -556,11 +584,12 @@ def main():
         if rank == 0:
             sampler.start()
         launches0 = L.b200z_launch_count()
-        res = fn(L, cores) if args.config == 3 else fn(L, cores, world, rank, dist if world > 1 else None)
+        ranks = () if args.config == 3 else (world, rank, dist if world > 1 else None)
+        res = fn(L, cores, *ranks, reps=args.steps)
         launches = L.b200z_launch_count() - launches0
         clocks = sampler.stop() if rank == 0 else None
         if rank == 0:
-            line = {"metric": res.pop("metric"), "value": res.pop("value"), "unit": res.pop("unit"), "n_gpus": world, "steps": 3,
+            line = {"metric": res.pop("metric"), "value": res.pop("value"), "unit": res.pop("unit"), "n_gpus": world, "steps": args.steps,
                     "warmup": 1, "ms_per_step": res.pop("ms_per_step"), "higher_is_better": True, "scaling": res.pop("scaling", "strong"),
                     "vs_baseline": None, "dtype": "u8", "data": "synthetic", "config": {"workload": res.pop("workload")},
                     "gpu_launches": int(launches), "clocks": clocks}
@@ -700,6 +729,8 @@ def main():
         dist.all_gather(allc, mine)
         gathered_ok = all(zlib.crc32(piece(r, c)) == int(allc[r][c]) for r in range(world) for c in range(NCH))
         assert gathered_ok, "the gathered stream differs from what its owners decoded"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, host_full, st, ol, us)
     del host_full
 
     # per-kernel breakdown (separate pass so event records do not sit inside the headline region)

@@ -1,4 +1,4 @@
-import csv, io, subprocess, sys
+import csv, io, os, subprocess, sys
 rep=sys.argv[1]
 raw = subprocess.run(["ncu","-i",rep,"--page","source","--csv","--print-source","cuda,sass","--kernel-name","regex:k_inflate_fast"],capture_output=True,text=True).stdout
 rows=list(csv.reader(io.StringIO(raw)))
@@ -15,7 +15,7 @@ for r in rows:
     else:
         a=lines.setdefault(-1,[0,0]); a[0]+=s; a[1]+=e
 # find phase boundaries by grepping the source
-src=open('/root/repo/archive_b200/csrc/inflate_fast.cuh').read().split('\n')
+src=open(os.path.join(os.path.dirname(os.path.abspath(__file__)),'..','archive_b200','csrc','inflate_fast.cuh')).read().split('\n')
 marks=[]
 def find(s):
     for i,l in enumerate(src):
