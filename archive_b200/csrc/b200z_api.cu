@@ -265,6 +265,24 @@ static int run_batch_on_staged(const uint64_t *in_off, const uint32_t *in_len, c
   return B200Z_OK;
 }
 
+cudaError_t copy_slots_to_host(uint8_t *host, const uint8_t *dev, uint64_t lo, const uint64_t *out_off, const uint32_t *out_cap,
+                               size_t n, cudaStream_t stream) {
+  std::vector<std::pair<uint64_t, uint64_t>> slots;
+  slots.reserve(n);
+  for (size_t u = 0; u < n; ++u)
+    if (out_cap[u]) slots.emplace_back(out_off[u], out_off[u] + out_cap[u]);
+  std::sort(slots.begin(), slots.end());
+  size_t i = 0;
+  while (i < slots.size()) {
+    const uint64_t a = slots[i].first;
+    uint64_t b = slots[i].second;
+    for (++i; i < slots.size() && slots[i].first <= b; ++i) b = std::max(b, slots[i].second);
+    const cudaError_t e = cudaMemcpyAsync(host + a, dev + (a - lo), b - a, cudaMemcpyDeviceToHost, stream);
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+
 static int stage_input(const uint8_t *in, size_t n) {
   CU(g.d_in.reserve(n + 64));
   if (n) CU(cudaMemcpyAsync(g.d_in.p, in, n, cudaMemcpyHostToDevice, g.stream));
@@ -2241,9 +2259,9 @@ void b200z_host_free(void *p) {
   if (p) cudaFreeHost(p);
 }
 
-size_t b200z_inflate_workspace_bytes(size_t n_units, size_t total_in_bytes, size_t total_out_cap) {
+size_t b200z_inflate_workspace_bytes(size_t n_units, size_t total_in_bytes, size_t out_extent) {
   (void)total_in_bytes;
-  return workspace_bytes(n_units, total_out_cap);
+  return workspace_bytes(n_units, out_extent);
 }
 
 int b200z_inflate_batch_device(const uint8_t *d_in_base, const uint64_t *d_in_off, const uint32_t *d_in_len,
@@ -2287,7 +2305,8 @@ int b200z_inflate_batch(const uint8_t *in_base, size_t in_bytes, const uint64_t 
   CU(g.d_out.reserve(out_bytes + 64));
   rc = run_batch_on_staged(in_off, in_len, out_off, out_cap, out_len, status, in_used, n_units, out_bytes);
   if (rc) return rc;
-  if (out_bytes) CU(cudaMemcpyAsync(out_base, g.d_out.p, out_bytes, cudaMemcpyDeviceToHost, g.stream));
+  // only the units' slots: the bytes between them are the caller's (the device buffer there holds earlier calls' data)
+  CU(copy_slots_to_host(out_base, (const uint8_t *)g.d_out.p, 0, out_off, out_cap, n_units, g.stream));
   CU(cudaStreamSynchronize(g.stream));
   return B200Z_OK;
 }

@@ -55,6 +55,10 @@ struct InflateBatch {
 };
 
 cudaError_t launch_inflate(const InflateBatch &b, cudaStream_t stream);
+// Device-to-host copy of the output slots of n units: host[out_off[u] .. +out_cap[u]) <- dev[out_off[u] - lo ..), one copy per
+// run of slots that touch or overlap.  The caller's bytes between slots are not written.
+cudaError_t copy_slots_to_host(uint8_t *host, const uint8_t *dev, uint64_t lo, const uint64_t *out_off, const uint32_t *out_cap,
+                               size_t n, cudaStream_t stream);
 cudaError_t launch_find_markers(const uint8_t *d_in, size_t n, unsigned long long *d_list, uint32_t *d_count, uint32_t cap,
                                 cudaStream_t stream);
 

@@ -231,7 +231,9 @@ int batch_multi(const uint8_t *in_base, const uint64_t *in_off, const uint32_t *
     b.ws = inflate_ws_carve(dv.ws.p, nu, ob);
     MCU(launch_inflate(b, dv.s));
     MCU(cudaMemcpyAsync(hm + nu * 24, dm + nu * 24, nu * 12, cudaMemcpyDeviceToHost, dv.s));
-    if (!gather && ob) MCU(cudaMemcpyAsync(out_base + s.out_lo, d_out, ob, cudaMemcpyDeviceToHost, dv.s));
+    // the device's slots only, not its min..max envelope: the bytes between slots (or other devices' slots inside the
+    // envelope when out_off is not monotone) are not this device's to write
+    if (!gather && ob) MCU(copy_slots_to_host(out_base, d_out, s.out_lo, out_off + s.u0, out_cap + s.u0, nu, dv.s));
   }
 #ifndef B200Z_EMU
   if (gather) {

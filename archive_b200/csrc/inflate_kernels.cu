@@ -445,13 +445,17 @@ cudaError_t launch_inflate(const InflateBatch &b, cudaStream_t stream) {
   // k_inflate_fast first (inflate_fast.cuh): a CTA per unit, everything in shared memory.  It finishes the clean units
   // whose output fits its window and flags them; the two exact kernels below then only see what is left.
   int after_fast = 0;
+  int fast_only = 0;
   {
     // B200Z_FAST=0 (read at every launch, so a process can time both) leaves everything to the exact pair.  Default on:
     // on the benchmark shape the kernel moves a fifth of the pair's DRAM bytes and takes 10.3 ms per GiB whatever the
     // data and the batch size, where the pair takes 9.3 ms on one rank's data and 13.5 on the others', and twice that
     // when a batch is launched in quarters (profiles/r2_summary.md, DESIGN.md K1f).
+    // B200Z_FAST=2 is a test and diagnostic mode: k_inflate_fast alone.  The units it leaves keep the out_len / status /
+    // in_used the caller put there and their output slots are not written, so a caller can see which units it finished.
     const char *fe = getenv("B200Z_FAST");
     const int fast_on = fe ? atoi(fe) : 1;
+    fast_only = fast_on == 2;
     if (fast_on && !b.count_only && b.ws.hist == 0 && b.ws.pieces != nullptr && b.ws.uscratch != nullptr) {
       static uint64_t attr_done = 0;  // one bit per device: function attributes belong to the device's context
       if (!((attr_done >> (cur_dev & 63)) & 1u)) {
@@ -481,6 +485,14 @@ cudaError_t launch_inflate(const InflateBatch &b, cudaStream_t stream) {
     }
   }
   if (g_prof) cudaEventRecord(pt.f, stream);
+  if (fast_only && after_fast) {
+    if (g_prof) {
+      cudaEventRecord(pt.b, stream);
+      cudaEventRecord(pt.c, stream);
+      g_prof_events.push_back(pt);
+    }
+    return cudaSuccess;
+  }
   if (b.ws.hist)
     k_inflate_decode<true><<<blocks, B200Z_DECODE_THREADS, smem, stream>>>(b.in_base, b.in_off, b.in_len, b.out_off, b.out_cap, b.ws,
                                                                          b.out_len, b.status, b.in_used, (uint32_t)b.n_units, upw,

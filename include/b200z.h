@@ -212,15 +212,22 @@ void b200z_file_last_stats(uint32_t *n_segments, uint32_t *n_whole);
 /* ---- batched independent units (what the kernels run) --------------------------------- */
 /* n_units raw DEFLATE streams: unit u reads in_base[in_off[u] .. +in_len[u]) and writes
  * out_base[out_off[u] .. +out_cap[u]).  Per unit: out_len, status (B200Z_U_*), in_used.
- * Host-pointer variant: copies in, runs, copies out (the end-to-end path).                  */
+ * Host-pointer variant: copies in, runs, copies out (the end-to-end path).  Only the units'
+ * slots are copied out: bytes of out_base between slots are left as the caller had them.    */
 int b200z_inflate_batch(const uint8_t *in_base, size_t in_bytes, const uint64_t *in_off,
                         const uint32_t *in_len, uint8_t *out_base, size_t out_bytes,
                         const uint64_t *out_off, const uint32_t *out_cap, uint32_t *out_len,
                         int32_t *status, uint32_t *in_used, size_t n_units);
 /* Device-pointer variant: every pointer is device memory on the b200z_init device; work is
  * enqueued on `cuda_stream` (a cudaStream_t, NULL = the library's stream) and NOT synchronised.
- * `workspace` must hold b200z_inflate_workspace_bytes(...) bytes.                           */
-size_t b200z_inflate_workspace_bytes(size_t n_units, size_t total_in_bytes, size_t total_out_cap);
+ * `workspace` must hold b200z_inflate_workspace_bytes(...) bytes.  Its third argument is the
+ * EXTENT of the output layout, max over u of out_off[u] + out_cap[u] -- not the sum of the caps:
+ * the workspace mirrors the output layout, gaps included.
+ * Test and diagnostic mode: with B200Z_FAST=2 in the environment (read at every call) only the
+ * shared-memory kernel runs.  A unit it does not finish keeps the out_len / status / in_used
+ * values the caller put there, and its output slot is not written.  B200Z_FAST=0 runs only the
+ * exact kernels; the default (1) runs both, the exact ones on what the first leaves.         */
+size_t b200z_inflate_workspace_bytes(size_t n_units, size_t total_in_bytes, size_t out_extent);
 int b200z_inflate_batch_device(const uint8_t *d_in_base, const uint64_t *d_in_off,
                                const uint32_t *d_in_len, uint8_t *d_out_base,
                                const uint64_t *d_out_off, const uint32_t *d_out_cap,
